@@ -10,6 +10,8 @@ Contract: `python bench.py --gpus N --steps K --warmup W [--impl reference]` pri
   * `roofline` = the dominant kernel's algorithmic bytes / its CUDA-event duration against MEASURED_PEAKS.json;
   * `cpu_baseline` / `--impl reference` = the CPU oracle (a port of the reference; the reference itself needs
     OpenCV/g2o and cannot be built here) timed on this box's host cores on a bounded sample of the same workload.
+  * `--dump-outputs DIR` writes what the last timed step returned (keypoints, descriptors, match pairs, its last local-BA window)
+    as DIR/<name>.npy; the inputs are seeded, so two builds run with the same arguments can be compared output for output.
 """
 import argparse
 import ctypes as C
@@ -54,7 +56,11 @@ def parse_args():
     ap.add_argument("--no-lba", action="store_true")
     ap.add_argument("--no-tracking", action="store_true", help="skip the second workload (device-resident track_local_map chain)")
     ap.add_argument("--lba-every", type=int, default=16, help="one local-BA window (50 keyframes / 10k landmarks) per this many frames")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write what the last timed step computed as DIR/<name>.npy")
+    args = ap.parse_args()
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of --impl b200")
+    return args
 
 
 # ---------------------------------------------------------------------------------------------------------------------
@@ -298,7 +304,7 @@ def main():
         lba_problem = synth.make_ba_problem(50, 10, 10000, seed=rank, model="stereo")
         lba_handles = [optimize.local_bundle_adjuster(device=local_rank) for _ in range(LBA_INFLIGHT)]
         lba_pool = ThreadPoolExecutor(LBA_INFLIGHT)
-    lba_state = {"launches": 0, "windows": 0, "pending": 0, "next": 0, "ref": None}
+    lba_state = {"launches": 0, "windows": 0, "pending": 0, "next": 0, "ref": None, "last": None}
     lba_inflight = []   # (future, handle index)
 
     def lba_prep(hidx, n):
@@ -324,6 +330,7 @@ def main():
     def lba_dispatch(n):
         hidx = lba_state["next"]
         lba_state["next"] = (hidx + 1) % LBA_INFLIGHT
+        lba_state["last"] = (hidx, n)
         for item in [it for it in lba_inflight if it[1] == hidx]:   # the handle's previous batch must be done
             lba_collect(item[0])
             lba_inflight.remove(item)
@@ -414,6 +421,13 @@ def main():
     last = sets[(step_no[0] - 1) & 1]
     n_kp = last.counts[1:].cpu().numpy()
     n_mt = last.n_pairs.cpu().numpy()
+    if args.dump_outputs and rank == 0:
+        lba_last = None
+        if n_lba:
+            prep = lba_preps[lba_state["last"]]
+            w = prep["n"] - 1
+            lba_last = (prep["pose"][w], prep["pts"][w], prep["outl"][w][:prep["arr"][w].n_edges])
+        dump_outputs(args.dump_outputs, last.kps[1:].cpu().numpy(), last.desc[1:].cpu().numpy(), n_kp, last.pairs.cpu().numpy(), n_mt, lba_last)
     value = multi_gpu.frames_per_second(B, args.steps, world, ms_total)
     repeat_stats = {"repeats": REPEATS, "ms_per_step": [m / args.steps for m in rep_ms], "median": ms_total / args.steps,
                     "min": min(rep_ms) / args.steps, "p10": float(np.percentile(rep_ms, 10)) / args.steps, "max": max(rep_ms) / args.steps}
@@ -701,6 +715,35 @@ def main():
     if world > 1:
         dist.destroy_process_group()
     return 0
+
+
+DUMP_LIMIT_BYTES = 60 << 20        # the whole dump, .npy headers included, stays under 64 MB
+
+
+def dump_outputs(out_dir, kps, desc, counts, pairs, n_pairs, lba):
+    """Write what one step returns to its caller as DIR/<name>.npy (float32; the local-BA window in float64), so that two builds can be
+    compared output for output.  Per frame: its keypoints (x, y, size, angle, response, octave), rBRIEF descriptors (one byte per
+    column) and (frame, previous frame) match pairs, concatenated in frame order; `frames` lists the frames written.  If all frames
+    would exceed DUMP_LIMIT_BYTES, a fixed, seeded sample of frames is written.  lba: (pose_cw, points, outlier flags) of the step's
+    last local-BA window, or None."""
+    counts, n_pairs = counts.astype(np.int64), n_pairs.astype(np.int64)
+    lba_bytes = sum(a.size * 8 for a in lba) if lba is not None else 0
+    frame_bytes = 4 * (counts * (6 + 32) + n_pairs * 2 + 3)
+    frames = np.arange(len(counts))
+    if frame_bytes.sum() + lba_bytes > DUMP_LIMIT_BYTES:
+        order = np.random.default_rng(0).permutation(len(counts))
+        frames = np.sort(order[:np.searchsorted(np.cumsum(frame_bytes[order]), DUMP_LIMIT_BYTES - lba_bytes, side="right")])
+    kp = np.concatenate([kps[f, :counts[f]] for f in frames])
+    kp[:, 5] = kp[:, 5].view(np.int32)          # the octave column holds int32 bits
+    out = {"frames": frames, "keypoint_counts": counts[frames], "keypoints": kp,
+           "descriptors": np.concatenate([desc[f, :counts[f]] for f in frames]),
+           "match_counts": n_pairs[frames], "match_pairs": np.concatenate([pairs[f, :n_pairs[f]] for f in frames])}
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a.astype(np.float32))
+    if lba is not None:
+        for name, a in zip(("lba_pose_cw", "lba_points", "lba_outliers"), lba):
+            np.save(os.path.join(out_dir, name + ".npy"), a.astype(np.float64))
 
 
 def bind_to_gpu_numa_node(torch, local_rank):

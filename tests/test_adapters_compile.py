@@ -1,10 +1,11 @@
 """The reference-side adapters (stella_vslam_b200/host/reference_adapters/*.cc) are the bindings a maintainer drops into the
-reference's src/ tree.  They cannot be LINKED here (Eigen, OpenCV, g2o, yaml-cpp, spdlog are not in this image), but they can be
-type-checked against the reference's REAL headers: `g++ -fsyntax-only` with /root/reference/src on the include path and minimal
+reference's src/ tree.  They cannot be LINKED without Eigen, OpenCV, g2o, yaml-cpp and spdlog, but they can be type-checked against
+the reference's REAL headers: `g++ -fsyntax-only` with a stella_vslam checkout's src/ on the include path and minimal
 declaration-only stand-ins (tests/cpp/stubs/) for the third-party headers those include.  That catches what VERDICT r1 asked for:
 signature drift against the reference interface, missing overrides, wrong member names.
 
-CPU test, runs only where /root/reference exists (the build container); skipped on the GPU box."""
+The type check needs the reference's headers, which this repository does not carry: it runs where REF_SRC holds them and skips
+elsewhere.  The other checks need nothing outside the repository and always run."""
 import glob
 import os
 import shutil
@@ -16,9 +17,6 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 REF_SRC = "/root/reference/src"
 ADAPTERS = sorted(glob.glob(os.path.join(ROOT, "stella_vslam_b200", "host", "reference_adapters", "*.cc")))
 
-pytestmark = pytest.mark.skipif(not os.path.isdir(REF_SRC) or shutil.which("g++") is None,
-                                reason="needs the reference headers and g++ (build container only)")
-
 
 def test_every_adapter_is_listed():
     names = {os.path.basename(p) for p in ADAPTERS}
@@ -26,6 +24,8 @@ def test_every_adapter_is_listed():
             "area_b200.cc", "bow_tree_b200.cc", "local_bundle_adjuster_b200.cc", "pose_optimizer_b200.cc", "global_bundle_adjuster_b200.cc", "track_local_map_b200.cc"} <= names
 
 
+@pytest.mark.skipif(not os.path.isdir(REF_SRC) or shutil.which("g++") is None,
+                    reason="needs the reference headers and g++")
 @pytest.mark.parametrize("src", ADAPTERS, ids=[os.path.basename(p) for p in ADAPTERS])
 def test_adapter_type_checks_against_reference_headers(src):
     cmd = ["g++", "-std=c++17", "-fsyntax-only", "-Wall", "-Wno-unused", "-Wno-sign-compare", "-DUSE_B200",
